@@ -12,6 +12,7 @@ channels@RT = samples/s / 48000.
   python bench.py --workload msk1200                        BASELINE configs[1]: 1024-channel continuous 1200 bps MSK, Eb/N0 8 dB
   python bench.py --workload burst1200x2048                 BASELINE configs[3]: the burst recording x2048, random frequency offsets
   python bench.py --workload mix16384 [--scaling strong]    BASELINE configs[4]: 10.5k OQPSK + 8400 bps C-channel mix, sharded
+  python bench.py ... --dump-outputs DIR                    also write what the last timed step decoded as DIR/<name>.npy
 
 Prints ONE JSON line (rank 0). `value` = device-timed, input resident in HBM; `e2e` = through the C ABI with HOST
 buffers (H2D of the PCM and D2H of the decoded signal units inside the timed region).
@@ -63,7 +64,15 @@ def parse():
     ap.add_argument("--streams", type=int, default=1, help="continuous workloads: split a GPU's channels into this many batches, each on its own CUDA stream "
                     "(the demodulator epoch of one batch then overlaps the estimator epoch of another)")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"], help="mix16384: weak = 2048 channels per GPU, strong = 16384 in total")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="continuous workloads: write what the last timed step decoded (signal units, CRC flags, DCD, loop state) "
+                    "as DIR/<name>.npy, so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.workload not in MODES):
+        ap.error("--dump-outputs applies to --impl ours with a continuous workload (%s)" % ", ".join(MODES))
+    return a
 
 
 # ----------------------------------------------------------------------------- synthetic input
@@ -306,11 +315,12 @@ class Pipeline:
         self.stream = stream
         self.stride = self.pcm.stride(0)
 
-    def step_device(self):
+    def step_device(self, keep_sus=False):
         self.batch.write_device(self.pcm.data_ptr(), STEP_SAMPLES, self.stride)
         self.layer.process_batch(self.batch)
         self.layer.tick(self.batch)
-        self.layer.discard_sus()          # results stay on the device for the HBM-resident measurement
+        if not keep_sus:
+            self.layer.discard_sus()      # results stay on the device for the HBM-resident measurement
 
     @property
     def launches(self):
@@ -320,8 +330,9 @@ class Pipeline:
         self.batch.close(); self.layer.close()
 
 
-def timed_steps(pipes, stream, steps, warmup, rank, local, dev):
-    """W warm-up steps, then exactly K steps between CUDA events on the launching stream; max over ranks."""
+def timed_steps(pipes, stream, steps, warmup, rank, local, dev, keep_last=False):
+    """W warm-up steps, then exactly K steps between CUDA events on the launching stream; max over ranks.
+    keep_last: the signal units of the last timed step stay queued for read_sus instead of being discarded."""
     import torch
     from jaero_b200 import shard
     clocks = ClockSampler(local)
@@ -341,9 +352,9 @@ def timed_steps(pipes, stream, steps, warmup, rank, local, dev):
     e0.record(stream)
     for so in others:
         so.wait_event(e0)                 # no batch starts before e0 ...
-    for _ in range(steps):
+    for k in range(steps):
         for p in pipes:
-            p.step_device()
+            p.step_device(keep_sus=keep_last and k == steps - 1)
     for so in others:
         ej = torch.cuda.Event(); ej.record(so); stream.wait_event(ej)   # ... and e1 fires when every batch is done
     e1.record(stream)
@@ -377,6 +388,43 @@ def roofline_block(mode, prof, C, ms_local, peaks):
                  "achieved": ach2, "frac": ach2 / peak, "avg_epoch_ms": prof["cfe_ms"] / max(1, prof["cfe_runs"]), "share_of_step": prof["cfe_ms"] / ms_local},
                 {"kernel": "whole step (all kernels)", "alg_bytes_per_sample": m["alg"] + ALG_K2, "achieved": step_ach, "frac": step_ach / peak}],
             "note": "per-channel fp64 feedback loop: bound by dependent-issue latency, not HBM (DESIGN.md section 5); K1a's own algorithmic bytes exclude the estimator's frame traffic, which is K2's"}
+
+
+DUMP_LIMIT = 64 << 20                 # bytes --dump-outputs may write
+
+
+def dump_outputs(out_dir, pipes):
+    """What the last timed step handed a caller of the P-channel path, one .npy per array (float32 / float64): the decoded
+    signal units of every channel concatenated in channel order (su_*, channel index in su_channel, per-channel count in
+    su_count), the DCD flag and cumulative SU counters per channel, and the demodulator's loop state per channel (state_*).
+    If the signal units would exceed DUMP_LIMIT, a fixed seeded sample of channels is kept (listed in su_channels_kept)."""
+    recs, counts = [], []
+    for p in pipes:
+        r, c = p.layer.read_sus_raw()
+        recs.append(r); counts.append(c)
+    rec = np.concatenate(recs); cnt = np.concatenate(counts).astype(np.int64)
+    n_ch = len(cnt)
+    keep = np.arange(n_ch)
+    per_su = 4 * (12 + 4)                                         # float32 bytes + crc_ok, index, frame, channel
+    if int(cnt.sum()) * per_su > DUMP_LIMIT // 2:
+        n_keep = max(1, int(n_ch * (DUMP_LIMIT // 2) // (int(cnt.sum()) * per_su)))
+        keep = np.sort(np.random.default_rng(0x4A4145).choice(n_ch, size=n_keep, replace=False))
+    sel = np.concatenate([np.stack([np.full(cnt[c], c), np.arange(cnt[c])], 1) for c in keep]).astype(np.int64).reshape(-1, 2)
+    r = rec[sel[:, 0], sel[:, 1]]
+    st = [s for p in pipes for s in p.batch.status()]
+    dcd, tot, ok = (np.concatenate([p.layer.stats()[i] for p in pipes]) for i in range(3))
+    arrays = {"su_bytes": r[:, :12].astype(np.float32), "su_crc_ok": r[:, 12].astype(np.float32),
+              "su_index_in_frame": r[:, 13].astype(np.float32),
+              "su_frame": (r[:, 14].astype(np.int32) | (r[:, 15].astype(np.int32) << 8)).astype(np.float32),
+              "su_channel": sel[:, 0].astype(np.float32), "su_count": cnt.astype(np.float32), "su_channels_kept": keep.astype(np.float32),
+              "dcd": dcd.astype(np.float32), "su_total": tot.astype(np.float64), "su_crc_ok_total": ok.astype(np.float64)}
+    for k in st[0]:
+        if k != "reserved":
+            arrays["state_" + k] = np.array([s[k] for s in st], dtype=np.float64)
+    assert sum(v.nbytes for v in arrays.values()) <= DUMP_LIMIT
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 # ----------------------------------------------------------------------------- workloads
@@ -433,7 +481,9 @@ def run_continuous(a, mode):
     pipes = [Pipeline(mode, Cg, ch0 + g * Cg, ebn0, envs_t, dev, local, streams[g]) for g in range(G)]
     pipe = pipes[0]
     torch.cuda.synchronize()
-    ms, ms_local, launches, profs, clk = timed_steps(pipes, stream, a.steps, a.warmup, rank, local, dev)
+    ms, ms_local, launches, profs, clk = timed_steps(pipes, stream, a.steps, a.warmup, rank, local, dev, keep_last=bool(a.dump_outputs))
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, pipes)
     st = [p.layer.stats() for p in pipes]
     dcd, su_tot, su_ok = (np.concatenate([x[i] for x in st]) for i in range(3))
     total_samples = float(C) * STEP_SAMPLES * a.steps * world

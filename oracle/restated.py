@@ -38,6 +38,7 @@ def lib():
         L.jor_rrc_design.argtypes = [d, i, d, d, vp, i]
         L.jor_trig_tables.argtypes = [vp, vp]; L.jor_qround.argtypes = [d]
         L.jor_fft.argtypes = [i, i, vp, vp]
+        L.jor_jfastfir_rrc.argtypes = [d, i, d, d, i, vp, l]
         L.jor_cfe_new.restype = vp; L.jor_cfe_new.argtypes = [i, d, d, d]
         L.jor_cfe_process.restype = d; L.jor_cfe_process.argtypes = [vp, vp, vp, vp]
         L.jor_cfe_bigchange.argtypes = [vp]; L.jor_cfe_free.argtypes = [vp]

@@ -79,6 +79,18 @@ void jor_free(void *hv) { OrHandle *h = (OrHandle *)hv; delete h->oq; delete h->
 
 int jor_rrc_design(double alpha, int firsize, double Fs, double symbol_freq, double *out, int cap)
 { std::vector<double> p = rrc_design(alpha, firsize, Fs, symbol_freq); int n = (int)p.size(); for (int i = 0; i < n && i < cap; i++) out[i] = p[i]; return n; }
+// restated JFastFir over a restated RRC kernel, configured as jref_jfastfir_rrc (oracle/ref_driver.cpp)
+void jor_jfastfir_rrc(double alpha, int firsize, double Fs, double symbol_freq, int nfft, double *inout_ri, long n)
+{
+    std::vector<double> pts = rrc_design(alpha, firsize, Fs, symbol_freq);
+    QVector<double> qp((int)pts.size());
+    for (size_t i = 0; i < pts.size(); i++) qp[(int)i] = pts[i];
+    JFastFir fir; fir.SetKernel(qp, nfft);
+    std::vector<JFastFir::cpx_type> v(n);
+    for (long i = 0; i < n; i++) v[i] = JFastFir::cpx_type(inout_ri[2 * i], inout_ri[2 * i + 1]);
+    fir.update(v.data(), (int)n);
+    for (long i = 0; i < n; i++) { inout_ri[2 * i] = v[i].real(); inout_ri[2 * i + 1] = v[i].imag(); }
+}
 void jor_trig_tables(double *s, double *c) { for (int i = 0; i < WTSIZE; i++) { s[i] = trig().SinWT[i]; c[i] = trig().CosWT[i]; } }
 int jor_qround(double d) { return jor::qRound(d); }
 void jor_fft(int n, int inverse, const double *in_ri, double *out_ri)

@@ -13,13 +13,11 @@ def pytest_configure(config):
 
 
 def _ensure_oracle():
-    """Build the CPU oracle libraries if they are missing (checker only, never the product)."""
+    """Build the CPU oracle library if it is missing (checker only, never the product). The reference build (oracle/_ref) is
+    not needed: its results are stored under tests/golden (tests/ref_pins.py)."""
     orc = os.path.join(ROOT, "oracle", "_build", "libjaero_oracle.so")
     if not os.path.exists(orc):
         subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "oracle"], check=True, capture_output=True)
-    refso = os.path.join(ROOT, "oracle", "_ref", "libjaero_ref.so")
-    if not os.path.exists(refso) and os.path.isdir("/root/reference/JAERO"):
-        subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True, capture_output=True)
 
 
 @pytest.fixture(scope="session", autouse=True)

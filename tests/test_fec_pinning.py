@@ -2,7 +2,8 @@
 helper classes compiled verbatim from JAERO/aerol.h:283-895 + aerol.cpp:523-902,2505-2524 (oracle/ref_fec_driver.cpp ->
 oracle/_ref/libjaero_ref_fec.so): CRC-16 (bytes and bits), scrambler, interleaver, puncturing, the three unique-word
 detectors and the R/T packet decoder RTChannelDeleaveFECScram (trial de-interleave + Viterbi + descramble + CRC at every
-candidate length). Random inputs, recorded soft bits and known-answer packets."""
+candidate length). Random inputs, recorded soft bits and known-answer packets. The reference's results on these inputs are
+stored in tests/golden/ref_pins.json (tests/ref_pins.py), so the tests need neither the reference nor oracle/_ref."""
 import ctypes
 import os
 
@@ -11,9 +12,9 @@ import pytest
 
 from conftest import ROOT, load_excerpt, synthetic_r_packet_stream
 from oracle import restated
+from ref_pins import RECORD, pinned, same
 
 SO = os.path.join(ROOT, "oracle", "_ref", "libjaero_ref_fec.so")
-pytestmark = pytest.mark.skipif(not os.path.exists(SO), reason="oracle/_ref/libjaero_ref_fec.so not built (needs /root/reference)")
 UW = 0xE15AE893
 C_PRE1, C_PRE2 = 216866263330005, 3012071630031408          # aerol.cpp:953-954
 
@@ -24,6 +25,9 @@ def _p(a):
 
 @pytest.fixture(scope="module")
 def F():
+    """the reference build, loaded only to record its results (ref_pins.RECORD)"""
+    if not RECORD:
+        return None
     L = ctypes.CDLL(SO)
     L.jfec_rt_new.restype = ctypes.c_void_p
     for n in ("jfec_rt_free", "jfec_rt_reset"):
@@ -48,11 +52,10 @@ def R():
 
 def test_crc16_bytes_and_bits(F, R):
     rng = np.random.default_rng(1)
-    for n in (1, 10, 12, 17, 19, 64):
-        for _ in range(50):
-            b = rng.integers(0, 256, size=n, dtype=np.uint8)
-            assert F.jfec_crc_bytes(_p(b), n) == R.jor_crc16(_p(b), n)
+    blocks = [rng.integers(0, 256, size=n, dtype=np.uint8) for n in (1, 10, 12, 17, 19, 64) for _ in range(50)]
+    assert same([R.jor_crc16(_p(b), len(b)) for b in blocks], "fec/crc16_bytes", lambda: [F.jfec_crc_bytes(_p(b), len(b)) for b in blocks])
     from jaero_b200 import synth
+    words = []
     for nbits in (8 * 19, 8 * 12, 48 + 96 * 3):
         for k in range(60):
             body = rng.integers(0, 2, size=nbits - 16).astype(np.int32)
@@ -61,18 +64,22 @@ def test_crc16_bytes_and_bits(F, R):
             bits = np.concatenate([body, np.array([(c >> i) & 1 for i in range(16)], dtype=np.int32)]).astype(np.int32)
             if k % 3 == 0:
                 bits[rng.integers(0, nbits)] ^= 1
-            assert F.jfec_crc_bits_check(_p(bits), nbits) == R.jor_pin_crc_bits_check(_p(bits), nbits)
+            words.append(bits)
+    assert same([R.jor_pin_crc_bits_check(_p(w), len(w)) for w in words], "fec/crc16_bits",
+                lambda: [F.jfec_crc_bits_check(_p(w), len(w)) for w in words])
     good = np.concatenate([np.zeros(136, dtype=np.int32), np.array([(synth.crc16(np.zeros(17, dtype=np.uint8)) >> i) & 1 for i in range(16)], dtype=np.int32)])
-    assert F.jfec_crc_bits_check(_p(good), 152) == 1 == R.jor_pin_crc_bits_check(_p(good), 152)
+    assert pinned("fec/crc16_bits_good", lambda: F.jfec_crc_bits_check(_p(good), 152)) == 1 == R.jor_pin_crc_bits_check(_p(good), 152)
 
 
 def test_scrambler_sequence_and_piecewise_update(F, R):
     seq = np.zeros(5000, dtype=np.int32)
     R.jor_pin_scrambler(_p(seq), 5000)
     sizes = np.array([288, 288, 1, 999, 2496, 928], dtype=np.int32)
-    bits = np.zeros(int(sizes.sum()), dtype=np.int32)                 # scrambling zeros returns the sequence itself
-    F.jfec_scramble(_p(bits), _p(sizes), len(sizes))
-    assert np.array_equal(bits, seq)
+    def ref():
+        bits = np.zeros(int(sizes.sum()), dtype=np.int32)             # scrambling zeros returns the sequence itself
+        F.jfec_scramble(_p(bits), _p(sizes), len(sizes))
+        return bits
+    assert same(seq, "fec/scrambler", ref)
     from jaero_b200 import synth
     assert np.array_equal(synth.scrambler_sequence(5000), seq.astype(np.uint8))
 
@@ -84,16 +91,21 @@ def test_deinterleaver_matches_reference(F, R, cols):
         block = rng.integers(0, 256, size=64 * cols).astype(np.int32)
         if setsize != cols:
             block = np.concatenate([block, rng.integers(0, 256, size=64 * (setsize - cols)).astype(np.int32)])
-        ref = np.zeros(64 * setsize, dtype=np.uint8)
-        n = F.jfec_deinterleave_ba(_p(block), len(block), setsize, cols, _p(ref))
+        def ref():
+            out = np.zeros(64 * setsize, dtype=np.uint8)
+            n = F.jfec_deinterleave_ba(_p(block), len(block), setsize, cols, _p(out))
+            return [n >= 64 * cols, out[:64 * cols]]
         got = np.zeros(64 * cols, dtype=np.uint8)
         R.jor_deinterleave(_p(np.ascontiguousarray(block[:64 * cols])), cols, _p(got))
-        assert n >= 64 * cols and np.array_equal(ref[:64 * cols], got)
+        assert same([True, got], "fec/deinterleave_%d_%d" % (cols, setsize), ref)
     # and the generator's interleaver is the reference's
     from jaero_b200 import synth
-    x = rng.integers(0, 2, size=64 * cols).astype(np.int32); o = np.zeros(64 * cols, dtype=np.int32)
-    assert F.jfec_interleave(_p(x), len(x), cols, _p(o)) == 64 * cols
-    assert np.array_equal(o, synth.interleave(x.astype(np.uint8), cols).astype(np.int32))
+    x = rng.integers(0, 2, size=64 * cols).astype(np.int32)
+
+    def ref_il():
+        o = np.zeros(64 * cols, dtype=np.int32)
+        return [F.jfec_interleave(_p(x), len(x), cols, _p(o)), o]
+    assert same([64 * cols, synth.interleave(x.astype(np.uint8), cols)], "fec/interleave_%d" % cols, ref_il)
 
 
 def test_c_channel_block_deinterleave_and_depuncture(F, R):
@@ -102,15 +114,17 @@ def test_c_channel_block_deinterleave_and_depuncture(F, R):
     frame = rng.integers(0, 256, size=4096).astype(np.int32)
     got = np.zeros(6000, dtype=np.uint8)
     ng = R.jor_pin_c_code_order(_p(frame), _p(got))
-    dele = []
-    for b in range(16):
-        o = np.zeros(64 * 95, dtype=np.uint8)
-        n = F.jfec_deinterleave_ba(_p(np.ascontiguousarray(frame[256 * b:256 * b + 256])), 256, 4, 4, _p(o))
-        dele.append(o[:256].copy()); assert n == 256
-    src = np.concatenate(dele); sizes = np.array([len(src)], dtype=np.int32)
-    ref = np.zeros(6000, dtype=np.uint8)
-    nr = F.jfec_depuncture(_p(src), _p(sizes), 1, 4, _p(ref))
-    assert nr == ng and np.array_equal(ref[:nr], got[:ng])
+    def ref():
+        dele = []
+        for b in range(16):
+            o = np.zeros(64 * 95, dtype=np.uint8)
+            n = F.jfec_deinterleave_ba(_p(np.ascontiguousarray(frame[256 * b:256 * b + 256])), 256, 4, 4, _p(o))
+            dele.append(o[:256].copy()); assert n == 256
+        src = np.concatenate(dele); sizes = np.array([len(src)], dtype=np.int32)
+        out = np.zeros(6000, dtype=np.uint8)
+        nr = F.jfec_depuncture(_p(src), _p(sizes), 1, 4, _p(out))
+        return [nr, out[:nr]]
+    assert same([ng, got[:ng]], "fec/c_code_order", ref)
 
 
 @pytest.mark.parametrize("kind,tol", [(0, 0), (1, 0), (3, 4), (2, 6)])
@@ -134,13 +148,15 @@ def test_unique_word_detectors_on_random_and_recorded_bits(F, R, kind, tol):
     pieces.append((soft > 0).astype(np.int32))
     bits = np.ascontiguousarray(np.concatenate(pieces))
     n = len(bits)
-    o1 = np.zeros(n, dtype=np.int32); i1 = np.zeros(n, dtype=np.int32); o2 = np.zeros(n, dtype=np.int32); i2 = np.zeros(n, dtype=np.int32)
     ref_kind = {0: 0, 1: 1, 3: 1, 2: 2}[kind]
-    F.jfec_detect(ref_kind, UW if kind != 2 else C_PRE1, C_PRE2, 32 if kind != 2 else 52, tol, _p(bits), n, _p(o1), _p(i1))
+
+    def ref():
+        o1 = np.zeros(n, dtype=np.int32); i1 = np.zeros(n, dtype=np.int32)
+        F.jfec_detect(ref_kind, UW if kind != 2 else C_PRE1, C_PRE2, 32 if kind != 2 else 52, tol, _p(bits), n, _p(o1), _p(i1))
+        return [o1, int(o1.sum()), i1 if kind else []]
+    o2 = np.zeros(n, dtype=np.int32); i2 = np.zeros(n, dtype=np.int32)
     R.jor_pin_detect(kind, tol, _p(bits), n, _p(o2), _p(i2))
-    assert np.array_equal(o1, o2) and o1.sum() >= 3
-    if kind:
-        assert np.array_equal(i1, i2)
+    assert same([o2, int(o2.sum()), i2 if kind else []], "fec/detect_%d_%d" % (kind, tol), ref) and o2.sum() >= 3
 
 
 def _rt_run(L, new, reset, update, info, free, fb, soft, msk):
@@ -159,6 +175,12 @@ def _rt_run(L, new, reset, update, info, free, fb, soft, msk):
     return res
 
 
+def _rt_key(res):
+    """what the two decoders must agree on: every report's position, result code, length and number of SUs, and the payload
+    bytes of every packet"""
+    return [list(x[:4]) + [x[4] if x[1] & 1 else b""] for x in res]
+
+
 @pytest.mark.parametrize("fb", [1200, 10500])
 def test_rt_packet_decoder_matches_reference_class(F, R, fb):
     """RTChannelDeleaveFECScram::update / updateMSK (aerol.h:631-877) against RTChannelOracle::rt_update / rt_updateMSK: the result
@@ -175,14 +197,10 @@ def test_rt_packet_decoder_matches_reference_class(F, R, fb):
             body = np.clip(body + rng.normal(0, 40, size=len(body)), 0, 255).astype(np.int16)
         streams.append(body.astype(np.int32))
     streams.append(rng.integers(0, 256, size=64 * 12).astype(np.int32))
-    for soft in streams:
-        a = _rt_run(F, F.jfec_rt_new, F.jfec_rt_reset, F.jfec_rt_update, F.jfec_rt_info, F.jfec_rt_free, None, soft, msk)
+    for k, soft in enumerate(streams):
+        a = lambda: _rt_key(_rt_run(F, F.jfec_rt_new, F.jfec_rt_reset, F.jfec_rt_update, F.jfec_rt_info, F.jfec_rt_free, None, soft, msk))
         b = _rt_run(R, R.jor_pin_rt_new, R.jor_pin_rt_reset, R.jor_pin_rt_update, R.jor_pin_rt_info, R.jor_pin_rt_free, fb, soft, msk)
-        assert [x[:4] for x in a] == [x[:4] for x in b]
-        for x, y in zip(a, b):
-            if x[1] & 1:                                             # a packet: the payload bytes too
-                assert x[4] == y[4]
-    assert any(x[1] == 3 for x in a) or True
+        assert same(_rt_key(b), "fec/rt_decoder_%d_%d" % (fb, k), a)
 
 
 def test_rt_t_packets_from_the_burst_recording(F, R):
@@ -207,8 +225,8 @@ def test_rt_t_packets_from_the_burst_recording(F, R):
         body = seg[pos:]
         if inv:
             body = np.where(body == 128, 128, 255 - body)
-        a = _rt_run(F, F.jfec_rt_new, F.jfec_rt_reset, F.jfec_rt_update, F.jfec_rt_info, F.jfec_rt_free, None, body, 1)
+        a = lambda: _rt_key(_rt_run(F, F.jfec_rt_new, F.jfec_rt_reset, F.jfec_rt_update, F.jfec_rt_info, F.jfec_rt_free, None, body, 1))
         b = _rt_run(R, R.jor_pin_rt_new, R.jor_pin_rt_reset, R.jor_pin_rt_update, R.jor_pin_rt_info, R.jor_pin_rt_free, 1200, body, 1)
-        assert [x[:4] for x in a] == [x[:4] for x in b] and all(x[4] == y[4] for x, y in zip(a, b) if x[1] & 1)
+        assert same(_rt_key(b), "fec/rt_recording_%d" % k, a)
         tried += 1
     assert tried >= 2

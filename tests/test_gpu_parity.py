@@ -603,19 +603,25 @@ def test_rt_channel_known_answer_r_packets(fb):
         assert np.array_equal(got[c][0]["bytes"][:17], payloads[c]) and len(got[c][0]["bytes"]) == 19
 
 
+# The reference's demodulator on the committed first 12 s of the 10.5k recording, framed by the restated P-channel layer and
+# reassembled by the reference's own code, gives exactly the first 520 CRC-valid signal units and the first 11 records (6 of
+# them ACARS) of what it gives on the whole 240 s recording (tools/make_reasm_golden.py --excerpt).
+EXCERPT_SUS, EXCERPT_RECORDS = 520, 11
+
+
 def test_recording_to_acars_end_to_end():
-    """240 s 10.5k recording -> device demodulator -> device P-channel frame layer -> host reassembly == the ACARS records the
-    reference's own demodulator + reassembly code produce (tests/golden/reasm_golden.json, tools/make_reasm_golden.py)."""
+    """12 s of the 10.5k recording -> device demodulator -> device P-channel frame layer -> host reassembly == the signal units
+    and ACARS records the reference's own demodulator + reassembly code produce (tests/golden/reasm_golden.json and
+    reasm_su_streams.npz, made from the whole recording by tools/make_reasm_golden.py)."""
     import json
     import reasm_synth
     jb = _import()
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "pcm_full", "oqpsk_10500.npy")
-    if not os.path.exists(path):
-        pytest.skip("full-length recording fixture not present (git-ignored; made by tools/make_fixtures.py)")
-    pcm = np.load(path)
-    with open(os.path.join(os.path.dirname(path), "..", "reasm_golden.json")) as fh:
-        want = json.load(fh)["p_recording_10500"]["records"]
-    want_sus = reasm_synth.unpack_stream(np.load(os.path.join(os.path.dirname(path), "..", "reasm_su_streams.npz"))["p_recording_10500"])
+    gold = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    pcm = load_excerpt("oqpsk_10500")
+    with open(os.path.join(gold, "reasm_golden.json")) as fh:
+        want = json.load(fh)["p_recording_10500"]["records"][:EXCERPT_RECORDS]
+    want_sus = reasm_synth.unpack_stream(np.load(os.path.join(gold, "reasm_su_streams.npz"))["p_recording_10500"])[:EXCERPT_SUS]
+    assert sum(1 for w in want if w["kind"] == 0 and not w["nonacars"]) == 6
     kw = dict(fb=10500, freq_center=5760, lockingbw=10500, fft_power=14, signalthreshold=0.65, afc=True)
     b = jb.DemodBatch("oqpsk", 2, **kw)
     pc = jb.PChannelBatch(2, 10500)

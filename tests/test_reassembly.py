@@ -2,8 +2,9 @@
 
 Golden records come from the reference's own code (JAERO/aerol.cpp:4-487 compiled verbatim, oracle/ref_reasm_driver.cpp)
 run by tools/make_reasm_golden.py over (1) the CRC-valid P-channel signal units the reference demodulator produces from
-the 240 s 10.5k recording, and (2) seeded synthetic streams (tests/reasm_synth.py). When oracle/_ref is present the
-reference is also run live on fresh random streams."""
+the 240 s 10.5k recording, and (2) seeded synthetic streams (tests/reasm_synth.py); for further random streams the
+reference's results are stored as digests (tests/ref_pins.py)."""
+import hashlib
 import json
 import os
 
@@ -12,6 +13,7 @@ import pytest
 
 import jaero_b200
 import reasm_synth
+from ref_pins import digest, pinned
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(HERE, "golden")
@@ -110,30 +112,51 @@ def test_pop_with_small_buffer():
     r.close()
 
 
+_FIELDS = ("aesid", "gesid", "qno", "refno", "seqno", "nooct", "mode", "tak", "bi", "nonacars", "downlink", "valid", "hastext", "moretocome")
+
+
+def _canon_ref(w):
+    """the parts of a reference record that _same compares, as JSON-able values"""
+    if w["kind"] != 0:
+        return [w["kind"], w["message"]]
+    return [w["kind"], w["message"]] + [int(w[k]) for k in _FIELDS] + [w["label"], w["reg"], len(w["userdata"]) // 2]
+
+
+def _canon_product(g):
+    if g["kind"] != 0:
+        return [g["kind"], g["text"].hex()]
+    return [g["kind"], g["text"].hex()] + [int(g[k]) for k in _FIELDS] + [g["label"].hex(), g["reg"].hex(), g["userdata_len"]]
+
+
+def _records_digest(canon):
+    return [len(canon), hashlib.sha256(json.dumps(canon).encode()).hexdigest()]
+
+
 @pytest.mark.parametrize("seed", [101, 102, 103])
 def test_reassembly_matches_reference_live(seed):
-    """fresh random streams, reference run here (skipped where oracle/_ref was not built)"""
-    from oracle import ref
-    if not ref.RefReasm.available():
-        pytest.skip("oracle/_ref/libjaero_ref_reasm.so not built")
+    """fresh random streams against the reference's reassembly run on them (oracle/_ref/libjaero_ref_reasm.so), whose return
+    codes and records are stored as digests in tests/golden/ref_pins.json"""
     stream = reasm_synth.p_stream(seed, burst=bool(seed & 1), n_msgs=50) + reasm_synth.r_stream(seed + 1, 40) + reasm_synth.garbage_stream(seed + 2, 1500)
-    rr = ref.RefReasm()
-    want_rc = []
-    for e in stream:
-        if e[0] == "su":
-            want_rc.append(rr.push_su(e[1], e[2]))
-        elif e[0] == "r":
-            want_rc.append(rr.push_r(e[1], e[2]))
-        elif e[0] == "reset":
-            rr.reset(); want_rc.append(0)
-        else:
-            rr.short_frame(); want_rc.append(0)
-    want = rr.pop_all(); rr.close()
+
+    def run():
+        from oracle import ref
+        rr = ref.RefReasm()
+        want_rc = []
+        for e in stream:
+            if e[0] == "su":
+                want_rc.append(rr.push_su(e[1], e[2]))
+            elif e[0] == "r":
+                want_rc.append(rr.push_r(e[1], e[2]))
+            elif e[0] == "reset":
+                rr.reset(); want_rc.append(0)
+            else:
+                rr.short_frame(); want_rc.append(0)
+        want = rr.pop_all(); rr.close()
+        return [np.array(want_rc), _records_digest([_canon_ref(w) for w in want])]
     rcs, out, _ = _run_product(stream)
-    assert rcs == want_rc
-    assert len(out) == len(want)
-    for g, w in zip(out, want):
-        _same(g, w)
+    want_rc, want = pinned("reasm/live_%d" % seed, run)
+    assert digest(np.array(rcs)) == want_rc
+    assert _records_digest([_canon_product(g) for g in out]) == want
 
 
 @pytest.mark.parametrize("name", ["p_recording_10500", "p_recording_600", "rt_recording_burst_oqpsk_10500", "p_synthetic", "t_synthetic", "r_synthetic", "garbage"])

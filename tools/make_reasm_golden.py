@@ -6,7 +6,8 @@ libjaero_ref_reasm.so = JAERO/aerol.cpp:4-487 compiled verbatim) run over
   (3) seeded synthetic SU streams that exercise multi-block ACARS, interleaved sequences, lost SSUs, parity errors,
       R-channel 1/2/3-SU sequences and the garbage cases.
 The SU byte streams themselves are committed (tests/golden/reasm_su_streams.npz) so the tests need neither the
-recordings nor /root/reference. Build container only."""
+recordings nor the reference. Needs oracle/_ref and the full recordings (tools/make_fixtures.py); --excerpt needs only
+oracle/_ref and prints how much of the recording's golden the committed 12 s excerpt covers."""
 import json
 import os
 import sys
@@ -20,9 +21,10 @@ from oracle import ref, restated  # noqa: E402
 import reasm_synth  # noqa: E402  (tests/reasm_synth.py)
 
 
-def recording_sus(name="oqpsk_10500", kind="oqpsk", kw=None):
+def recording_sus(name="oqpsk_10500", kind="oqpsk", kw=None, pcm=None):
     import multiprocessing as mp
-    pcm = np.load(os.path.join(ROOT, "tests", "golden", "pcm_full", name + ".npy"))
+    if pcm is None:
+        pcm = np.load(os.path.join(ROOT, "tests", "golden", "pcm_full", name + ".npy"))
     kw = kw or dict(fb=10500, freq_center=5760, lockingbw=10500, fft_power=14, signalthreshold=0.65, afc=True)
     ctx = mp.get_context("spawn")
     with ctx.Pool(1) as pool:
@@ -74,7 +76,22 @@ def run_stream(stream):
     return rcs, out
 
 
-if __name__ == "__main__":
+def excerpt_prefix():
+    """The committed 12 s excerpt through the same chain: its CRC-valid SUs and reassembled records must be a prefix of the
+    whole recording's (tests/test_gpu_parity.py EXCERPT_SUS, EXCERPT_RECORDS)."""
+    import json
+    sus = recording_sus(pcm=np.load(os.path.join(ROOT, "tests", "golden", "oqpsk_10500_excerpt.npz"))["pcm"])
+    full = reasm_synth.unpack_stream(np.load(os.path.join(ROOT, "tests", "golden", "reasm_su_streams.npz"))["p_recording_10500"])
+    _, out = run_stream([("su", bytes(x), False) for x in sus])
+    with open(os.path.join(ROOT, "tests", "golden", "reasm_golden.json")) as fh:
+        gold = json.load(fh)["p_recording_10500"]["records"]
+    assert [bytes(x) for x in sus] == [e[1] for e in full[:len(sus)]] and out == gold[:len(out)]
+    print("EXCERPT_SUS, EXCERPT_RECORDS = %d, %d" % (len(sus), len(out)))
+
+
+if __name__ == "__main__" and sys.argv[1:] == ["--excerpt"]:
+    excerpt_prefix()
+elif __name__ == "__main__":
     streams = {}
     rec = recording_sus()
     streams["p_recording_10500"] = [("su", bytes(x), False) for x in rec]
