@@ -44,6 +44,16 @@ class AcarsRecord(ctypes.Structure):
                 ("flags", ctypes.c_uint8), ("userdata_len", ctypes.c_uint32), ("text_len", ctypes.c_uint32)]
 
 
+class ChanSettings(ctypes.Structure):
+    """jaero_chan_settings (include/jaero_b200.h)."""
+    _fields_ = [("iq_format", ctypes.c_int), ("reserved", ctypes.c_int), ("input_rate", ctypes.c_double),
+                ("output_rate", ctypes.c_double), ("audio_hz", ctypes.c_double), ("passband_hz", ctypes.c_double),
+                ("gain", ctypes.c_double)]
+
+
+IQ_FORMATS = {"cs16": 0, "cu8": 1}
+
+
 EXPORTS = ["jaero_last_error", "jaero_device_count", "jaero_batch_create", "jaero_batch_destroy", "jaero_batch_channels",
            "jaero_batch_write", "jaero_batch_write_device", "jaero_batch_sync", "jaero_batch_read_softbits",
            "jaero_batch_softbits_device", "jaero_batch_reset_softbits", "jaero_batch_set_dcd",
@@ -66,7 +76,9 @@ EXPORTS = ["jaero_last_error", "jaero_device_count", "jaero_batch_create", "jaer
            "jaero_cchannel_tick", "jaero_cchannel_read_frames", "jaero_cchannel_get_stats", "jaero_cchannel_launch_count",
            "jaero_ingest_create", "jaero_ingest_destroy", "jaero_ingest_message", "jaero_ingest_available", "jaero_ingest_flush",
            "jaero_reasm_create", "jaero_reasm_destroy", "jaero_reasm_reset", "jaero_reasm_short_frame", "jaero_reasm_push_su",
-           "jaero_reasm_push_r", "jaero_reasm_push_t_packet", "jaero_reasm_pending", "jaero_reasm_pop", "jaero_reasm_get_stats"]
+           "jaero_reasm_push_r", "jaero_reasm_push_t_packet", "jaero_reasm_pending", "jaero_reasm_pop", "jaero_reasm_get_stats",
+           "jaero_chan_taps", "jaero_chan_create", "jaero_chan_destroy", "jaero_chan_write", "jaero_chan_write_device",
+           "jaero_chan_output_device", "jaero_chan_read", "jaero_chan_set_stream", "jaero_chan_sync", "jaero_chan_launch_count"]
 
 
 def lib():
@@ -156,6 +168,14 @@ def lib():
         L.jaero_reasm_pending.argtypes = [vp]
         L.jaero_reasm_pop.argtypes = [vp, ctypes.POINTER(AcarsRecord), vp, sz]; L.jaero_reasm_pop.restype = ctypes.c_long
         L.jaero_reasm_get_stats.argtypes = [vp, vp, vp, vp, vp]
+        L.jaero_chan_taps.argtypes = [ctypes.POINTER(ChanSettings), vp, i]
+        L.jaero_chan_create.argtypes = [ctypes.POINTER(ChanSettings), i, vp, i, ctypes.POINTER(vp)]
+        L.jaero_chan_destroy.argtypes = [vp]; L.jaero_chan_destroy.restype = None
+        L.jaero_chan_write.argtypes = [vp, vp, sz]; L.jaero_chan_write_device.argtypes = [vp, vp, sz]
+        L.jaero_chan_output_device.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(sz), ctypes.POINTER(sz)]
+        L.jaero_chan_read.argtypes = [vp, vp, sz, ctypes.POINTER(sz)]
+        L.jaero_chan_set_stream.argtypes = [vp, vp]; L.jaero_chan_sync.argtypes = [vp]
+        L.jaero_chan_launch_count.argtypes = [vp]; L.jaero_chan_launch_count.restype = ctypes.c_int64
         _lib = L
     return _lib
 
@@ -711,6 +731,84 @@ class Reassembler:
     def close(self):
         if self.h:
             lib().jaero_reasm_destroy(self.h); self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _chan_settings(input_rate, output_rate, audio_hz, passband_hz, iq_format, gain):
+    if iq_format not in IQ_FORMATS:
+        raise JaeroError("iq_format must be one of %s" % sorted(IQ_FORMATS))
+    return ChanSettings(IQ_FORMATS[iq_format], 0, float(input_rate), float(output_rate), float(audio_hz), float(passband_hz), float(gain))
+
+
+def channelizer_taps(input_rate, output_rate=48000.0, audio_hz=12000.0, passband_hz=12000.0, iq_format="cs16", gain=1.0):
+    """The channelizer's low-pass h[0..T-1] (float64, unity DC gain), designed on the host; no device needed."""
+    s = _chan_settings(input_rate, output_rate, audio_hz, passband_hz, iq_format, gain)
+    T = lib().jaero_chan_taps(ctypes.byref(s), None, 0)
+    if T < 0:
+        _check(T)
+    h = np.zeros(T, dtype=np.float64)
+    lib().jaero_chan_taps(ctypes.byref(s), _p(h), T)
+    return h
+
+
+class Channelizer:
+    """One wideband complex IQ stream -> one real int16 audio row per channel (channel c's carrier moved to audio_hz at
+    output_rate), on the device. The rows feed DemodBatch.write_device(ptr, n, stride) as they are (see output_device)."""
+
+    def __init__(self, offsets_hz, input_rate, output_rate=48000.0, audio_hz=12000.0, passband_hz=12000.0, iq_format="cs16",
+                 gain=1.0, device=0):
+        s = _chan_settings(input_rate, output_rate, audio_hz, passband_hz, iq_format, gain)
+        off = np.ascontiguousarray(np.atleast_1d(np.asarray(offsets_hz, dtype=np.float64)))
+        self.h = ctypes.c_void_p()
+        self.n = len(off)
+        self.iq_format = iq_format
+        self.D = int(round(float(input_rate) / float(output_rate)))
+        _check(lib().jaero_chan_create(ctypes.byref(s), self.n, _p(off), device, ctypes.byref(self.h)))
+
+    def write(self, iq):
+        """iq: host array [n, 2] of int16 (cs16) or uint8 (cu8) I, Q pairs."""
+        iq = np.ascontiguousarray(iq)
+        want = np.int16 if self.iq_format == "cs16" else np.uint8
+        if iq.dtype != want or iq.ndim != 2 or iq.shape[1] != 2:
+            raise JaeroError("write expects a [n, 2] %s array" % np.dtype(want).name)
+        _check(lib().jaero_chan_write(self.h, _p(iq), iq.shape[0]))
+
+    def write_device(self, dev_ptr, n_iq):
+        """n_iq complex samples already in this GPU's memory (interleaved I, Q in the handle's format)."""
+        _check(lib().jaero_chan_write_device(self.h, ctypes.c_void_p(dev_ptr), int(n_iq)))
+
+    def output_device(self):
+        """(device pointer, samples per channel, channel stride) of the rows the last write produced; valid until the next write."""
+        a, n, st = ctypes.c_void_p(), ctypes.c_size_t(), ctypes.c_size_t()
+        _check(lib().jaero_chan_output_device(self.h, ctypes.byref(a), ctypes.byref(n), ctypes.byref(st)))
+        return a.value, n.value, st.value
+
+    def read(self):
+        """int16 [n_channels, n] copy of the rows the last write produced (synchronises)."""
+        _, n, _ = self.output_device()
+        out = np.zeros((self.n, max(n, 1)), dtype=np.int16)
+        got = ctypes.c_size_t()
+        _check(lib().jaero_chan_read(self.h, _p(out), out.shape[1], ctypes.byref(got)))
+        return out[:, :got.value]
+
+    def set_stream(self, cuda_stream):
+        _check(lib().jaero_chan_set_stream(self.h, ctypes.c_void_p(cuda_stream)))
+
+    def sync(self):
+        _check(lib().jaero_chan_sync(self.h))
+
+    @property
+    def launches(self):
+        return lib().jaero_chan_launch_count(self.h)
+
+    def close(self):
+        if self.h:
+            lib().jaero_chan_destroy(self.h); self.h = None
 
     def __del__(self):
         try:

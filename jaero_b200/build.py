@@ -19,6 +19,7 @@ UNITS = [
     ("rtchannel.cu", []),
     ("cchannel.cu", []),
     ("reassembly.cu", []),
+    ("channelizer.cu", []),                  # restates no reference arithmetic: FMA contraction is allowed
     ("prefilter.cu", ["-fmad=false"]),
     ("burst.cu", ["-fmad=false"]),
     ("demod_kernels.cu", ["-fmad=false"]),

@@ -266,3 +266,44 @@ def offset_replicas(pcm, offsets_hz, Fs=48000.0):
 def replica_offsets(r0, r1, span_hz=300.0, seed0=0xB0057):
     """df_r = U(-span, span) from seed seed0 + r (cfg 4: span 300 Hz)."""
     return np.array([np.random.default_rng(seed0 + r).uniform(-span_hz, span_hz) for r in range(r0, r1)])
+
+
+def wideband_iq(envelopes, offsets_hz, input_rate, env_rate=48000.0, amplitudes=None, ebn0_db=None, fb=10500.0, seed=0,
+                iq_format="cs16", noise_ref=0):
+    """Complex baseband IQ at input_rate carrying each circular envelope (oqpsk_envelope / msk_envelope, unit power, at
+    env_rate) at its offset, plus complex AWGN, quantised as an SDR delivers it: [n, 2] int16 (cs16) or uint8 (cu8, the
+    rtl_sdr format, x = ((u - 127.5) + j(v - 127.5)) * 256). Amplitudes (RMS, in cs16 LSB) default to 1000.
+    Each envelope is interpolated by zero-padding its FFT, so the result still loops seamlessly when every offset is a
+    multiple of env_rate / len(envelope). Noise: per-component variance N0 * input_rate / 2 with
+    N0 = P / fb / 10^(ebn0_db / 10) of carrier `noise_ref` (P = its amplitude squared, fb its bit rate)."""
+    up = float(input_rate) / float(env_rate)
+    U = int(round(up))
+    assert abs(up - U) < 1e-9 and U >= 1, "input_rate must be an integer multiple of env_rate"
+    L = len(envelopes[0])
+    assert all(len(e) == L for e in envelopes)
+    n = L * U
+    amps = np.full(len(envelopes), 1000.0) if amplitudes is None else np.asarray(amplitudes, dtype=np.float64)
+    fbs = np.broadcast_to(np.asarray(fb, dtype=np.float64), (len(envelopes),))
+    t = np.arange(n, dtype=np.float64)
+    x = np.zeros(n, dtype=np.complex128)
+    for env, off, a in zip(envelopes, offsets_hz, amps):
+        E = np.fft.fft(np.asarray(env, dtype=np.complex128))
+        Z = np.zeros(n, dtype=np.complex128)
+        h = L // 2
+        Z[:h] = E[:h]
+        Z[n - (L - h):] = E[h:]
+        if L % 2 == 0:                                            # split the Nyquist bin so the result stays band-limited
+            Z[h] = 0.5 * E[h]; Z[n - h] = 0.5 * E[h]
+        y = np.fft.ifft(Z) * U
+        x += a * y * np.exp(2j * np.pi * float(off) * t / float(input_rate))
+    if ebn0_db is not None:
+        rng = np.random.default_rng(seed)
+        n0 = amps[noise_ref] ** 2 / fbs[noise_ref] / (10.0 ** (ebn0_db / 10.0))
+        sd = np.sqrt(n0 * float(input_rate) / 2.0)
+        x += rng.normal(0.0, sd, n) + 1j * rng.normal(0.0, sd, n)
+    out = np.stack([x.real, x.imag], axis=1)
+    if iq_format == "cs16":
+        return np.clip(np.rint(out), -32768, 32767).astype(np.int16)
+    if iq_format == "cu8":
+        return np.clip(np.rint(out / 256.0 + 127.5), 0, 255).astype(np.uint8)
+    raise ValueError("iq_format must be cs16 or cu8")
