@@ -13,6 +13,11 @@ COMMON = ["-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "-Xcompiler",
 # rounds exactly as the CPU reference does (x86-64 has no implicit FMA contraction).
 UNITS = [
     ("capi.cu", []),
+    ("capi_batch.cu", []),
+    ("capi_burst.cu", []),
+    ("capi_frames.cu", []),
+    ("capi_ingest.cu", []),
+    ("host_design.cpp", []),                 # host C++ only: nvcc hands it to the host compiler with the flags above
     ("viterbi.cu", []),
     ("cfe.cu", []),
     ("pchannel.cu", []),
@@ -36,11 +41,11 @@ def _stale(target, deps):
 def build(force=False, verbose=False):
     objdir = os.path.join(HERE, "_obj")
     os.makedirs(objdir, exist_ok=True)
-    hdrs = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h", ".cu"))]
+    hdrs = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h", ".cu", ".cpp"))]
     hdrs.append(os.path.join(os.path.dirname(HERE), "include", "jaero_b200.h"))
     objs = []
     for src, extra in UNITS:
-        obj = os.path.join(objdir, src.replace(".cu", ".o"))
+        obj = os.path.join(objdir, os.path.splitext(src)[0] + ".o")
         objs.append(obj)
         if force or _stale(obj, hdrs):
             cmd = [NVCC] + ARCH + COMMON + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", os.path.join(CSRC, src), "-o", obj]

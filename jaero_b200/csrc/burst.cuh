@@ -75,5 +75,6 @@ int hilbert_block_launch(const HilbertStream &h, int n_channels, int first_block
 int burst_front_launch(const BurstParams &p, long long sample0, int n, cudaStream_t s);
 int burst_trident_launch(const BurstParams &p, double2 *work_a, double2 *work_b, const double2 *tw16k, double *absbuf, cudaStream_t s, long long *launches);
 int burst_back_launch(const BurstParams &p, long long sample0, int n, int new_write, cudaStream_t s);
+int burst_trident_fft_launch(const BurstParams &p, const int *d_ev_list, int n_events, double2 *wa, double2 *wb, const double2 *tw, cudaStream_t s);
 
 } // namespace jb

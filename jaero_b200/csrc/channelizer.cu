@@ -9,7 +9,7 @@
 // (shared by all channels; channels carry no other state). chan_ddc_kernel runs k in a fixed ascending order for every
 // output, so each output's sum does not depend on how the input was cut into writes.
 #include "../../include/jaero_b200.h"
-#include "common.cuh"
+#include "handle.cuh"
 #include <cmath>
 #include <cstring>
 #include <new>
@@ -181,12 +181,13 @@ struct jaero_chan {
     double gain;
     uint32_t inc_a;
     cudaStream_t stream, own_stream;
+    HandleAllocs allocs;
     float2 *d_G;
     uint32_t *d_inc;
-    float2 *d_x[2]; size_t x_cap[2]; int cur; long long last_n;   // ping-pong sample buffers, H history + last write
+    GrowBuffer<float2> x[2]; int cur; long long last_n;            // ping-pong sample buffers, H history + last write
     bool have_prev;
-    uint8_t *d_raw; size_t raw_cap;                                 // staging for host writes
-    int16_t *d_out; size_t out_cap, stride, n_out;
+    GrowBuffer<uint8_t> raw;                                        // staging for host writes
+    GrowBuffer<int16_t> out; size_t stride, n_out;                  // [C][stride]
     long long n_in;                                                 // input samples so far
     int64_t launches;
 };
@@ -208,7 +209,7 @@ void jaero_chan_destroy(jaero_chan *c)
     if (!c) return;
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
-    cudaFree(c->d_G); cudaFree(c->d_inc); cudaFree(c->d_x[0]); cudaFree(c->d_x[1]); cudaFree(c->d_raw); cudaFree(c->d_out);
+    c->allocs.free_all(); c->x[0].release(); c->x[1].release(); c->raw.release(); c->out.release();
     if (c->own_stream) cudaStreamDestroy(c->own_stream);
     delete c;
 }
@@ -225,14 +226,11 @@ int jaero_chan_create(const jaero_chan_settings *s, int n_channels, const double
         if (!std::isfinite(o) || std::fabs(o) + 0.5 * s->passband_hz > 0.5 * s->input_rate) {
             set_error("jaero_chan_create: channel " + std::to_string(c) + " does not fit inside the input band"); return JAERO_E_ARG; }
     }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess) { cudaGetLastError(); ndev = 0; }
-    if (device < 0 || device >= ndev) { set_error("jaero_chan_create: no such CUDA device (there is no CPU fallback)"); return JAERO_E_CUDA; }
-    JB_CUDA(cudaSetDevice(device));
-    jaero_chan *c = new (std::nothrow) jaero_chan();
-    if (!c) { set_error("out of host memory"); return JAERO_E_ARG; }
-    memset(c, 0, sizeof *c);
-    c->device = device; c->C = n_channels; c->T = T; c->D = D; c->fmt = s->iq_format; c->gain = s->gain;
+    NewHandle<jaero_chan> nh(jaero_chan_destroy);
+    int r = nh.open(device, "jaero_chan_create"); if (r) return r;
+    jaero_chan *c = nh.h;
+    c->own_stream = c->stream;
+    c->C = n_channels; c->T = T; c->D = D; c->fmt = s->iq_format; c->gain = s->gain;
     c->Cpad = (n_channels + TILE_C - 1) / TILE_C * TILE_C;
     c->Tpad = (T + KC - 1) / KC * KC;
     c->H = c->Tpad - 1;
@@ -246,16 +244,9 @@ int jaero_chan_create(const jaero_chan_settings *s, int n_channels, const double
             double a = 2.0 * M_PI * (double)ph / 4294967296.0;
             G[(size_t)k * c->Cpad + ch] = make_float2((float)(h[k] * std::cos(a)), (float)(h[k] * std::sin(a)));
         }
-    int rc = JAERO_OK;
-    auto fail = [&](cudaError_t e, const char *what) { rc = cuda_fail(e, what, __FILE__, __LINE__); jaero_chan_destroy(c); return rc; };
-    cudaError_t e;
-    if ((e = cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking)) != cudaSuccess) return fail(e, "cudaStreamCreate");
-    c->stream = c->own_stream;
-    if ((e = cudaMalloc(&c->d_G, G.size() * sizeof(float2))) != cudaSuccess) return fail(e, "cudaMalloc(G)");
-    if ((e = cudaMalloc(&c->d_inc, inc.size() * sizeof(uint32_t))) != cudaSuccess) return fail(e, "cudaMalloc(inc)");
-    if ((e = cudaMemcpy(c->d_G, G.data(), G.size() * sizeof(float2), cudaMemcpyHostToDevice)) != cudaSuccess) return fail(e, "cudaMemcpy(G)");
-    if ((e = cudaMemcpy(c->d_inc, inc.data(), inc.size() * sizeof(uint32_t), cudaMemcpyHostToDevice)) != cudaSuccess) return fail(e, "cudaMemcpy(inc)");
-    *out = c;
+    if (c->allocs.upload(&c->d_G, G, c->stream) || c->allocs.upload(&c->d_inc, inc, c->stream)) return JAERO_E_CUDA;
+    JB_CUDA(cudaStreamSynchronize(c->stream));
+    *out = nh.release();
     return JAERO_OK;
 }
 
@@ -290,30 +281,21 @@ int jaero_chan_write_device(jaero_chan *c, const void *d_iq, size_t n)
     if (n == 0) return JAERO_OK;
     const int nb = 1 - c->cur;
     const size_t need = (size_t)c->H + n;
-    if (c->x_cap[nb] < need || (M > 0 && ((M + 7) & ~(size_t)7) > c->stride)) {
-        JB_CUDA(cudaStreamSynchronize(c->stream));
-        if (c->x_cap[nb] < need) {
-            cudaFree(c->d_x[nb]); c->d_x[nb] = 0; c->x_cap[nb] = 0;
-            JB_CUDA(cudaMalloc(&c->d_x[nb], need * sizeof(float2)));
-            c->x_cap[nb] = need;
-        }
-        size_t st = (M + 7) & ~(size_t)7;
-        if (st > c->stride) {
-            cudaFree(c->d_out); c->d_out = 0; c->out_cap = 0; c->stride = 0;
-            JB_CUDA(cudaMalloc(&c->d_out, st * c->C * sizeof(int16_t)));
-            c->stride = st; c->out_cap = st * c->C;
-        }
+    if (c->x[nb].reserve(need, c->stream)) return JAERO_E_CUDA;
+    if (M > 0) {
+        if (c->out.reserve(((M + 7) & ~(size_t)7) * c->C, c->stream)) return JAERO_E_CUDA;
+        c->stride = c->out.cap / c->C;
     }
     const long long tot = c->H + (long long)n;
     chan_convert_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, c->stream>>>(d_iq, c->fmt, (long long)n,
-                                                                              c->have_prev ? c->d_x[c->cur] : nullptr, c->last_n, c->H, c->d_x[nb]);
+                                                                              c->have_prev ? c->x[c->cur].ptr : nullptr, c->last_n, c->H, c->x[nb].ptr);
     JB_CUDA(cudaGetLastError());
     c->launches++;
     if (M > 0) {
         dim3 grid((unsigned)((M + TILE_M - 1) / TILE_M), (unsigned)(c->Cpad / TILE_C));
         const long long off0 = m_first * D - N0 + c->H;
-        chan_ddc_kernel<<<grid, THREADS, 0, c->stream>>>(c->d_G, c->Cpad, c->Tpad, c->C, c->d_x[nb], off0, c->D, (int)M,
-                                                         (unsigned long long)m_first, c->d_inc, c->inc_a, c->gain, c->d_out, c->stride);
+        chan_ddc_kernel<<<grid, THREADS, 0, c->stream>>>(c->d_G, c->Cpad, c->Tpad, c->C, c->x[nb].ptr, off0, c->D, (int)M,
+                                                         (unsigned long long)m_first, c->d_inc, c->inc_a, c->gain, c->out.ptr, c->stride);
         JB_CUDA(cudaGetLastError());
         c->launches++;
     }
@@ -329,20 +311,15 @@ int jaero_chan_write(jaero_chan *c, const void *iq, size_t n)
     if (n == 0) return jaero_chan_write_device(c, nullptr, 0);
     JB_CUDA(cudaSetDevice(c->device));
     const size_t bytes = n * (c->fmt == JAERO_IQ_CS16 ? 4 : 2);
-    if (bytes > c->raw_cap) {
-        JB_CUDA(cudaStreamSynchronize(c->stream));
-        cudaFree(c->d_raw); c->d_raw = 0; c->raw_cap = 0;
-        JB_CUDA(cudaMalloc(&c->d_raw, bytes));
-        c->raw_cap = bytes;
-    }
-    JB_CUDA(cudaMemcpyAsync(c->d_raw, iq, bytes, cudaMemcpyHostToDevice, c->stream));
-    return jaero_chan_write_device(c, c->d_raw, n);
+    if (c->raw.reserve(bytes, c->stream)) return JAERO_E_CUDA;
+    JB_CUDA(cudaMemcpyAsync(c->raw.ptr, iq, bytes, cudaMemcpyHostToDevice, c->stream));
+    return jaero_chan_write_device(c, c->raw.ptr, n);
 }
 
 int jaero_chan_output_device(jaero_chan *c, const int16_t **d_pcm, size_t *n_samples, size_t *channel_stride)
 {
     if (!c || !d_pcm || !n_samples || !channel_stride) { set_error("jaero_chan_output_device: null argument"); return JAERO_E_ARG; }
-    *d_pcm = c->d_out; *n_samples = c->n_out; *channel_stride = c->stride;
+    *d_pcm = c->out.ptr; *n_samples = c->n_out; *channel_stride = c->stride;
     return JAERO_OK;
 }
 
@@ -353,7 +330,7 @@ int jaero_chan_read(jaero_chan *c, int16_t *out, size_t cap, size_t *n_samples)
     JB_CUDA(cudaSetDevice(c->device));
     *n_samples = c->n_out;
     if (c->n_out)
-        JB_CUDA(cudaMemcpy2DAsync(out, cap * sizeof(int16_t), c->d_out, c->stride * sizeof(int16_t), c->n_out * sizeof(int16_t), c->C,
+        JB_CUDA(cudaMemcpy2DAsync(out, cap * sizeof(int16_t), c->out.ptr, c->stride * sizeof(int16_t), c->n_out * sizeof(int16_t), c->C,
                                   cudaMemcpyDeviceToHost, c->stream));
     JB_CUDA(cudaStreamSynchronize(c->stream));
     return JAERO_OK;

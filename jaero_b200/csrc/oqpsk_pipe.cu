@@ -77,7 +77,7 @@ oqpsk_pipe_kernel(const __grid_constant__ DemodParams p, const SegmentArgs a, co
     const int lane = threadIdx.x & 31;
     const int warp = (int)(threadIdx.x >> 5);
     // Which channel this lane carries. Channels are independent, so the library may seat them as it likes: it regroups them by
-    // symbol-timing phase (capi.cu, regroup) so that the 32 channels of a CTA strobe on the same samples - the expensive
+    // symbol-timing phase (capi_batch.cu, regroup) so that the 32 channels of a CTA strobe on the same samples - the expensive
     // carrier-update path of warps K1 / K2 then runs on one sample in nine instead of (some lane) on every sample. All state
     // stays indexed by channel; only the sample-rate rings, which are laid out by seat, move when the seating changes.
     const int seat = blockIdx.x * OQ_THREADS + lane;
@@ -110,7 +110,7 @@ oqpsk_pipe_kernel(const __grid_constant__ DemodParams p, const SegmentArgs a, co
             int countdown = LI(I_COUNTDOWN), countdown2 = LI(I_COUNTDOWN2);
             double est = 0.0;
             if (a.cfe_wait > 0) {
-                // The estimator of this trigger runs concurrently (capi.cu). Its result only enters the arithmetic below when
+                // The estimator of this trigger runs concurrently (capi_batch.cu). Its result only enters the arithmetic below when
                 // the channel is unlocked / has no carrier detect, and its state (y[], emptyingcountdown) is only touched by
                 // the AFC re-centre: channels in neither case proceed without it.
                 const bool recentre = (p.afc) && (mse < p.signalthreshold) && (fabs(m2.freq - mc.freq) > 3.0) && (countdown <= 0);
