@@ -334,35 +334,43 @@ int jaero_reasm_get_stats(const jaero_reasm *h, uint64_t *isus, uint64_t *messag
 /* ---- device channelizer: one wideband complex IQ stream -> per-channel real audio rows for the demodulator batches ----
  * The reference has no channelizer (it takes audio from a sound card or ZMQ), so this definition is the contract.
  * x[n] counted from the handle's first write at input_rate (cs16: I,Q as they are; cu8: x = ((I-127.5) + j(Q-127.5)) * 256).
- * D = input_rate / output_rate (integer >= 2). Phases are uint32 fractions of a cycle: inc_c = llround(offset_c / input_rate
- * * 2^32) mod 2^32, phi_c(n) = inc_c * n mod 2^32, inc_a = llround(audio_hz / output_rate * 2^32), psi(m) = inc_a * m mod 2^32.
- * h[0..T-1] is the Kaiser low-pass jaero_chan_taps returns (unity DC gain). Output m of channel c sits at input index m*D:
- *   a_c[m]   = sum_k h[k] x[mD-k] exp(-2 pi j phi_c(mD-k) / 2^32)              (x[n<0] = 0)
+ * Rate change: L/M = output_rate / input_rate in lowest terms, accepted when 1 <= L <= 64 and M >= 2L. L is the smallest of
+ * 1..64 for which r*L (r = input_rate / output_rate) lies within 1e-9 * r*L of an integer M; L = 1 is an integer ratio D = M.
+ * Phases are uint32 fractions of a cycle: inc_c = llround(offset_c / input_rate * 2^32) mod 2^32, phi_c(n) = inc_c * n
+ * mod 2^32, inc_a = llround(audio_hz / output_rate * 2^32), psi(m) = inc_a * m mod 2^32.
+ * h[0..T-1] is the Kaiser low-pass prototype jaero_chan_taps returns, designed at L * input_rate and scaled to sum L (unity
+ * DC gain in each of the L polyphase branches); h[j] = 0 for j >= T, Tp = ceil(T/L) taps per branch. Output m of channel c
+ * sits at input time mM/L: n_m = floor(mM/L), p_m = mM mod L,
+ *   a_c[m]   = sum_{k<Tp} h[kL + p_m] x[n_m - k] exp(-2 pi j phi_c(n_m - k) / 2^32)              (x[n<0] = 0)
  *   out_c[m] = saturate_int16(round_half_even(gain * Re{a_c[m] exp(2 pi j psi(m) / 2^32)}))
- * i.e. mix channel c to 0 Hz, low-pass, keep every D-th sample, move it to audio_hz, take the real part: the audio a
- * batch with freq_center = audio_hz and Fs = output_rate expects. Filter: f_p = passband_hz/2, f_s = min(2 audio_hz,
- * output_rate - 2 audio_hz) - f_p (nearest alias / real-part fold into the passband), A = 60 dB, beta = 0.1102 (A - 8.7),
- * T from Kaiser's estimate made odd (<= 8191), cutoff (f_p + f_s)/2, scaled to sum 1. */
+ * i.e. mix channel c to 0 Hz, resample by L/M (zero-stuff by L, low-pass at L*input_rate, keep every M-th sample), move it to
+ * audio_hz, take the real part: the audio a batch with freq_center = audio_hz and Fs = output_rate expects. With L = 1,
+ * n_m = mD and the sum runs over h[k] x[mD-k]. Filter: f_p = passband_hz/2, f_s = min(2 audio_hz, output_rate - 2 audio_hz)
+ * - f_p (nearest alias / real-part fold into the passband), A = 60 dB, beta = 0.1102 (A - 8.7), T from Kaiser's estimate at
+ * L * input_rate made odd (Tp <= 8191), cutoff (f_p + f_s)/2. */
 #define JAERO_IQ_CS16 0
 #define JAERO_IQ_CU8 1
-#define JAERO_CHAN_MAX_TAPS 8191
+#define JAERO_CHAN_MAX_TAPS 8191     /* per polyphase branch */
+#define JAERO_CHAN_MAX_PHASES 64     /* largest L */
 typedef struct jaero_chan_settings {
     int iq_format;                   /* JAERO_IQ_* */
     int reserved;
-    double input_rate, output_rate;  /* Hz; input_rate = D * output_rate, D integer >= 2 */
+    double input_rate, output_rate;  /* Hz; output_rate / input_rate = L/M, L <= 64, M >= 2L */
     double audio_hz;                 /* where each channel's centre lands in the audio (= the batch's freq_center) */
     double passband_hz;              /* two-sided width kept within 0.05 dB */
     double gain;
 } jaero_chan_settings;
 typedef struct jaero_chan jaero_chan;
-/* host only, no device: returns T (or a negative error), writes min(T, cap) taps; taps may be NULL */
+/* host only, no device: returns T (or a negative error), writes min(T, cap) taps of the prototype (sum L); taps may be NULL */
 int jaero_chan_taps(const jaero_chan_settings *s, double *taps, int cap);
+/* host only, no device: validates the settings as jaero_chan_taps does and returns the rate change L/M (either may be NULL) */
+int jaero_chan_ratio(const jaero_chan_settings *s, int *L, int *M);
 /* n_channels channels at offset_hz[c] from the IQ centre. Settings and offsets are validated before any device is touched. */
 int jaero_chan_create(const jaero_chan_settings *s, int n_channels, const double *offset_hz, int device_ordinal, jaero_chan **out);
 void jaero_chan_destroy(jaero_chan *c);
 int jaero_chan_write(jaero_chan *c, const void *iq, size_t n_iq);           /* HOST iq, n_iq complex samples */
 int jaero_chan_write_device(jaero_chan *c, const void *d_iq, size_t n_iq);  /* device iq; several handles may read the same buffer */
-/* The audio produced by the most recent write (every output m with mD inside the input so far), valid until the next write:
+/* The audio produced by the most recent write (every output m with n_m inside the input so far), valid until the next write:
  * d_pcm[ch * channel_stride + i], i < n_samples; 16-byte aligned base, stride a multiple of 8 (jaero_batch_write_device takes
  * it as is). Ordered on the handle's stream. */
 int jaero_chan_output_device(jaero_chan *c, const int16_t **d_pcm, size_t *n_samples, size_t *channel_stride);

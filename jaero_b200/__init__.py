@@ -78,7 +78,8 @@ EXPORTS = ["jaero_last_error", "jaero_device_count", "jaero_batch_create", "jaer
            "jaero_reasm_create", "jaero_reasm_destroy", "jaero_reasm_reset", "jaero_reasm_short_frame", "jaero_reasm_push_su",
            "jaero_reasm_push_r", "jaero_reasm_push_t_packet", "jaero_reasm_pending", "jaero_reasm_pop", "jaero_reasm_get_stats",
            "jaero_chan_taps", "jaero_chan_create", "jaero_chan_destroy", "jaero_chan_write", "jaero_chan_write_device",
-           "jaero_chan_output_device", "jaero_chan_read", "jaero_chan_set_stream", "jaero_chan_sync", "jaero_chan_launch_count"]
+           "jaero_chan_output_device", "jaero_chan_read", "jaero_chan_set_stream", "jaero_chan_sync", "jaero_chan_launch_count",
+           "jaero_chan_ratio"]
 
 
 def lib():
@@ -169,6 +170,7 @@ def lib():
         L.jaero_reasm_pop.argtypes = [vp, ctypes.POINTER(AcarsRecord), vp, sz]; L.jaero_reasm_pop.restype = ctypes.c_long
         L.jaero_reasm_get_stats.argtypes = [vp, vp, vp, vp, vp]
         L.jaero_chan_taps.argtypes = [ctypes.POINTER(ChanSettings), vp, i]
+        L.jaero_chan_ratio.argtypes = [ctypes.POINTER(ChanSettings), ctypes.POINTER(i), ctypes.POINTER(i)]
         L.jaero_chan_create.argtypes = [ctypes.POINTER(ChanSettings), i, vp, i, ctypes.POINTER(vp)]
         L.jaero_chan_destroy.argtypes = [vp]; L.jaero_chan_destroy.restype = None
         L.jaero_chan_write.argtypes = [vp, vp, sz]; L.jaero_chan_write_device.argtypes = [vp, vp, sz]
@@ -746,7 +748,8 @@ def _chan_settings(input_rate, output_rate, audio_hz, passband_hz, iq_format, ga
 
 
 def channelizer_taps(input_rate, output_rate=48000.0, audio_hz=12000.0, passband_hz=12000.0, iq_format="cs16", gain=1.0):
-    """The channelizer's low-pass h[0..T-1] (float64, unity DC gain), designed on the host; no device needed."""
+    """The channelizer's low-pass prototype h[0..T-1] (float64, designed at L * input_rate, sum L: unity DC gain in each
+    polyphase branch), designed on the host; no device needed."""
     s = _chan_settings(input_rate, output_rate, audio_hz, passband_hz, iq_format, gain)
     T = lib().jaero_chan_taps(ctypes.byref(s), None, 0)
     if T < 0:
@@ -756,9 +759,19 @@ def channelizer_taps(input_rate, output_rate=48000.0, audio_hz=12000.0, passband
     return h
 
 
+def channelizer_ratio(input_rate, output_rate=48000.0, audio_hz=12000.0, passband_hz=12000.0, iq_format="cs16", gain=1.0):
+    """(L, M) with output_rate / input_rate = L/M in lowest terms, as the channelizer accepts it (L <= 64, M >= 2L; L = 1 for
+    an integer ratio); validates every setting as channelizer_taps does. No device needed."""
+    s = _chan_settings(input_rate, output_rate, audio_hz, passband_hz, iq_format, gain)
+    Lr, Mr = ctypes.c_int(), ctypes.c_int()
+    _check(lib().jaero_chan_ratio(ctypes.byref(s), ctypes.byref(Lr), ctypes.byref(Mr)))
+    return Lr.value, Mr.value
+
+
 class Channelizer:
     """One wideband complex IQ stream -> one real int16 audio row per channel (channel c's carrier moved to audio_hz at
-    output_rate), on the device. The rows feed DemodBatch.write_device(ptr, n, stride) as they are (see output_device)."""
+    output_rate), on the device. The rows feed DemodBatch.write_device(ptr, n, stride) as they are (see output_device).
+    ratio is (L, M), output_rate / input_rate = L/M; D is the integer ratio M when L = 1, else None."""
 
     def __init__(self, offsets_hz, input_rate, output_rate=48000.0, audio_hz=12000.0, passband_hz=12000.0, iq_format="cs16",
                  gain=1.0, device=0):
@@ -767,8 +780,9 @@ class Channelizer:
         self.h = ctypes.c_void_p()
         self.n = len(off)
         self.iq_format = iq_format
-        self.D = int(round(float(input_rate) / float(output_rate)))
         _check(lib().jaero_chan_create(ctypes.byref(s), self.n, _p(off), device, ctypes.byref(self.h)))
+        self.ratio = channelizer_ratio(input_rate, output_rate, audio_hz, passband_hz, iq_format, gain)
+        self.D = self.ratio[1] if self.ratio[0] == 1 else None
 
     def write(self, iq):
         """iq: host array [n, 2] of int16 (cs16) or uint8 (cu8) I, Q pairs."""

@@ -1,16 +1,20 @@
 // Device channelizer (include/jaero_b200.h, "device channelizer"): one wideband complex IQ stream in, one real int16 audio
 // row per channel out, in the layout jaero_batch_write_device consumes.
 //
-// phi_c(mD - k) = phi_c(mD) - phi_c(k) holds exactly in uint32 phase arithmetic, so the mix-to-0-Hz, low-pass and decimate of
-// every channel is one complex matrix product shared by all channels:
-//   A[c][m] = sum_k G[c][k] X[k][m],   G[c][k] = h[k] e^{+2 pi j phi_c(k) / 2^32},   X[k][m] = x[mD - k],
-// followed per output by one rotation through (psi(m) - phi_c(mD)) mod 2^32, the gain, rounding and saturation.
-// G is built once at create (double, stored as float2); x is kept as float2 behind a copy of the last Tpad-1 input samples
-// (shared by all channels; channels carry no other state). chan_ddc_kernel runs k in a fixed ascending order for every
-// output, so each output's sum does not depend on how the input was cut into writes.
+// The rate change is L/M (L = 1 for an integer ratio D = M). Output m sits at input time mM/L: n_m = floor(mM/L), polyphase
+// branch p_m = mM mod L, taps h[kL + p_m]. phi_c(n - k) = phi_c(n) - phi_c(k) holds exactly in uint32 phase arithmetic, so the
+// mix-to-0-Hz, low-pass and resample of every channel is one complex matrix product per branch, shared by all channels:
+//   A[c][m] = sum_k G[p_m][k][c] X[k][m],   G[p][k][c] = h[kL + p] e^{+2 pi j phi_c(k) / 2^32},   X[k][m] = x[n_m - k],
+// followed per output by one rotation through (psi(m) - phi_c(n_m)) mod 2^32, the gain, rounding and saturation.
+// The outputs m = m_r + jL of one residue class share the branch and step through the input by exactly M, so each class is
+// an integer-stride decimation; one launch covers all classes (blockIdx.z). G is built once at create (double, stored as
+// float2); x is kept as float2 behind a copy of the last Tpad-1 input samples (shared by all channels; channels carry no
+// other state). chan_ddc_kernel runs k in a fixed ascending order for every output, so each output's sum does not depend
+// on how the input was cut into writes.
 #include "../../include/jaero_b200.h"
 #include "handle.cuh"
 #include <cmath>
+#include <algorithm>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -47,17 +51,27 @@ __global__ void chan_convert_kernel(const void *__restrict__ iq, int fmt, long l
     cur[i] = v;
 }
 
-// One block: TILE_C channels x TILE_M outputs. G is [Tpad][Cpad] (tap-major, zero beyond T and C); xb[pos] with
-// pos = off0 + j*D - k for local output j; out[c*stride + j].
+// One block: TILE_C channels x TILE_M outputs of residue class q = blockIdx.z, i.e. outputs m = m_first + q + jL. G is
+// [L][Tpad][Cpad] (branch-major, then tap-major, zero beyond Tp and C). The class starts at m_r = m_first + q, input index
+// n_r = floor(m_r Dm / L), branch p = m_r Dm mod L; its local output j reads xb[pos], pos = n_r + hist + j*Dm - k
+// (hist = H - N0: where input index n lies in xb), and goes to out[c*stride + q + j*L]. With L = 1 this is the integer-D
+// decimation: one class, p = 0, n_r = m_first * D.
 __global__ void __launch_bounds__(THREADS) chan_ddc_kernel(const float2 *__restrict__ G, int Cpad, int Tpad, int C,
-                                                           const float2 *__restrict__ xb, long long off0, int D, int M,
-                                                           unsigned long long m_first, const uint32_t *__restrict__ inc_c,
+                                                           const float2 *__restrict__ xb, long long hist, int Dm, int L,
+                                                           int n_out, unsigned long long m_first, const uint32_t *__restrict__ inc_c,
                                                            uint32_t inc_a, double gain, int16_t *__restrict__ out, size_t stride)
 {
     __shared__ float2 Gs[KC][TILE_C];
     __shared__ float2 Xs[KC][TILE_M + 1];
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-    const int c0 = blockIdx.y * TILE_C, j0 = blockIdx.x * TILE_M;
+    const int q = blockIdx.z, c0 = blockIdx.y * TILE_C, j0 = blockIdx.x * TILE_M;
+    const int M = (n_out - q + L - 1) / L;                                   // outputs of this class in this write
+    if (j0 >= M) return;
+    const unsigned long long m_r = m_first + q, t_r = m_r * (unsigned long long)Dm;
+    const unsigned long long n_r = t_r / (unsigned)L;
+    const int p = (int)(t_r % (unsigned)L);
+    const long long off0 = (long long)n_r + hist;
+    G += (size_t)p * Tpad * Cpad;
     float2 acc[RC][RM];
 #pragma unroll
     for (int i = 0; i < RC; i++)
@@ -73,7 +87,7 @@ __global__ void __launch_bounds__(THREADS) chan_ddc_kernel(const float2 *__restr
 #pragma unroll
         for (int r = 0; r < KC * TILE_M / THREADS; r++) {
             int e = tid + r * THREADS, kk = e % KC, mm = e / KC, j = j0 + mm;
-            Xs[kk][mm] = j < M ? xb[off0 + (long long)j * D - (k0 + kk)] : make_float2(0.f, 0.f);
+            Xs[kk][mm] = j < M ? xb[off0 + (long long)j * Dm - (k0 + kk)] : make_float2(0.f, 0.f);
         }
         __syncthreads();
 #pragma unroll
@@ -104,16 +118,15 @@ __global__ void __launch_bounds__(THREADS) chan_ddc_kernel(const float2 *__restr
         for (int j = 0; j < RM; j++) {
             int jj = j0 + tx + 16 * j;
             if (jj >= M) continue;
-            unsigned long long m = m_first + jj;
-            uint32_t phi = ic * (uint32_t)(m * (unsigned long long)D);   // phi_c(mD), mod 2^32
-            uint32_t psi = inc_a * (uint32_t)m;
+            uint32_t phi = ic * (uint32_t)(n_r + (unsigned long long)jj * Dm);   // phi_c(n_m), mod 2^32
+            uint32_t psi = inc_a * (uint32_t)(m_r + (unsigned long long)jj * L);
             int32_t th = (int32_t)(psi - phi);
             double s, co;
             sincospi((double)th * (1.0 / 2147483648.0), &s, &co);
             double v = gain * ((double)acc[i][j].x * co - (double)acc[i][j].y * s);
             v = rint(v);
             v = fmin(fmax(v, -32768.0), 32767.0);
-            out[(size_t)c * stride + jj] = (int16_t)v;
+            out[(size_t)c * stride + q + (size_t)jj * L] = (int16_t)v;
         }
     }
 }
@@ -129,34 +142,42 @@ double bessel_i0(double x)
     return sum;
 }
 
-// Validates the settings and designs h (scipy.signal.firwin(T, (f_p + f_s)/2, window=('kaiser', beta), fs=input_rate) with T
-// from kaiserord(60, (f_s - f_p) / (input_rate / 2)), made odd). Returns T or JAERO_E_ARG.
-int chan_design(const jaero_chan_settings *s, std::vector<double> *h, int *D_out)
+// Validates the settings, finds L/M = output_rate / input_rate in lowest terms (the smallest L in 1..64 for which r L,
+// r = input_rate / output_rate, is within 1e-9 r L of an integer M; M >= 2L) and designs the prototype h at L * input_rate:
+// scipy.signal.firwin(T, (f_p + f_s)/2, window=('kaiser', beta), fs=L*input_rate) * L with T from
+// kaiserord(60, (f_s - f_p) / (L*input_rate / 2)), made odd, and at most 8191 taps per branch (ceil(T/L)). Returns T or
+// JAERO_E_ARG.
+int chan_design(const jaero_chan_settings *s, std::vector<double> *h, int *L_out, int *M_out)
 {
     if (!s) { set_error("jaero_chan: null settings"); return JAERO_E_ARG; }
     if (s->iq_format != JAERO_IQ_CS16 && s->iq_format != JAERO_IQ_CU8) { set_error("jaero_chan: unknown iq_format"); return JAERO_E_ARG; }
     if (!std::isfinite(s->input_rate) || !std::isfinite(s->output_rate) || s->input_rate <= 0 || s->output_rate <= 0) {
         set_error("jaero_chan: input_rate and output_rate must be positive"); return JAERO_E_ARG; }
     double r = s->input_rate / s->output_rate;
-    double Dd = std::floor(r + 0.5);
-    if (std::fabs(r - Dd) > 1e-9 * r || Dd < 2 || Dd > 1e6) {
-        set_error("jaero_chan: input_rate / output_rate must be an integer D >= 2"); return JAERO_E_ARG; }
+    int L = 0;
+    double Md = 0;
+    for (int l = 1; l <= JAERO_CHAN_MAX_PHASES && !L; l++) {
+        double rl = r * l, m = std::floor(rl + 0.5);
+        if (std::fabs(rl - m) <= 1e-9 * rl) { L = l; Md = m; }
+    }
+    if (!L || Md < 2 * L || Md > 1e6 * L) {
+        set_error("jaero_chan: output_rate / input_rate must be L/M with L <= 64 and M >= 2L"); return JAERO_E_ARG; }
     if (!std::isfinite(s->audio_hz) || s->audio_hz <= 0 || s->audio_hz >= 0.5 * s->output_rate) {
         set_error("jaero_chan: audio_hz must lie in (0, output_rate/2)"); return JAERO_E_ARG; }
     if (!std::isfinite(s->passband_hz) || s->passband_hz <= 0) { set_error("jaero_chan: passband_hz must be positive"); return JAERO_E_ARG; }
     if (!std::isfinite(s->gain) || s->gain <= 0) { set_error("jaero_chan: gain must be positive and finite"); return JAERO_E_ARG; }
-    const double A = 60.0;
+    const double A = 60.0, fsamp = L * s->input_rate;
     double fp = 0.5 * s->passband_hz;
     double fs = std::fmin(2 * s->audio_hz, s->output_rate - 2 * s->audio_hz) - fp;
     if (!(fs > fp)) { set_error("jaero_chan: no transition band (f_s <= f_p): narrow the passband or move audio_hz"); return JAERO_E_ARG; }
-    double width = (fs - fp) / (0.5 * s->input_rate);
+    double width = (fs - fp) / (0.5 * fsamp);
     double numtaps = (A - 7.95) / 2.285 / (M_PI * width) + 1;
-    if (!(numtaps <= JAERO_CHAN_MAX_TAPS)) { set_error("jaero_chan: filter longer than 8191 taps"); return JAERO_E_ARG; }
+    if (!(numtaps <= (double)JAERO_CHAN_MAX_TAPS * L)) { set_error("jaero_chan: filter longer than 8191 taps per phase"); return JAERO_E_ARG; }
     int T = (int)std::ceil(numtaps);
     if (!(T & 1)) T++;
-    if (T > JAERO_CHAN_MAX_TAPS) { set_error("jaero_chan: filter longer than 8191 taps"); return JAERO_E_ARG; }
+    if ((T + L - 1) / L > JAERO_CHAN_MAX_TAPS) { set_error("jaero_chan: filter longer than 8191 taps per phase"); return JAERO_E_ARG; }
     if (h) {
-        const double beta = 0.1102 * (A - 8.7), cut = (fp + fs) / 2 / (0.5 * s->input_rate), alpha = 0.5 * (T - 1);
+        const double beta = 0.1102 * (A - 8.7), cut = (fp + fs) / 2 / (0.5 * fsamp), alpha = 0.5 * (T - 1);
         const double i0b = bessel_i0(beta);
         h->assign(T, 0.0);
         double sum = 0;
@@ -168,16 +189,17 @@ int chan_design(const jaero_chan_settings *s, std::vector<double> *h, int *D_out
             (*h)[n] = cut * sinc * w;
             sum += (*h)[n];
         }
-        for (int n = 0; n < T; n++) (*h)[n] /= sum;
+        for (int n = 0; n < T; n++) (*h)[n] = (*h)[n] / sum * L;   // sum L: unity DC gain in every branch
     }
-    if (D_out) *D_out = (int)Dd;
+    if (L_out) *L_out = L;
+    if (M_out) *M_out = (int)Md;
     return T;
 }
 
 } // namespace
 
 struct jaero_chan {
-    int device, C, Cpad, T, Tpad, H, D, fmt;
+    int device, C, Cpad, T, Tpad, H, L, M, fmt;                      // Tpad: taps per branch, ceil(T/L) rounded up to KC
     double gain;
     uint32_t inc_a;
     cudaStream_t stream, own_stream;
@@ -197,11 +219,21 @@ extern "C" {
 int jaero_chan_taps(const jaero_chan_settings *s, double *taps, int cap)
 {
     std::vector<double> h;
-    int T = chan_design(s, taps ? &h : nullptr, nullptr);
+    int T = chan_design(s, taps ? &h : nullptr, nullptr, nullptr);
     if (T < 0) return T;
     if (taps)
         for (int k = 0; k < T && k < cap; k++) taps[k] = h[k];
     return T;
+}
+
+int jaero_chan_ratio(const jaero_chan_settings *s, int *L, int *M)
+{
+    int l = 0, m = 0;
+    int T = chan_design(s, nullptr, &l, &m);
+    if (T < 0) return T;
+    if (L) *L = l;
+    if (M) *M = m;
+    return JAERO_OK;
 }
 
 void jaero_chan_destroy(jaero_chan *c)
@@ -218,8 +250,8 @@ int jaero_chan_create(const jaero_chan_settings *s, int n_channels, const double
 {
     if (!out || n_channels <= 0 || !offset_hz) { set_error("jaero_chan_create: bad argument (n_channels must be positive)"); return JAERO_E_ARG; }
     std::vector<double> h;
-    int D = 0;
-    int T = chan_design(s, &h, &D);
+    int L = 0, M = 0;
+    int T = chan_design(s, &h, &L, &M);
     if (T < 0) return T;
     for (int c = 0; c < n_channels; c++) {
         double o = offset_hz[c];
@@ -230,19 +262,24 @@ int jaero_chan_create(const jaero_chan_settings *s, int n_channels, const double
     int r = nh.open(device, "jaero_chan_create"); if (r) return r;
     jaero_chan *c = nh.h;
     c->own_stream = c->stream;
-    c->C = n_channels; c->T = T; c->D = D; c->fmt = s->iq_format; c->gain = s->gain;
+    c->C = n_channels; c->T = T; c->L = L; c->M = M; c->fmt = s->iq_format; c->gain = s->gain;
+    const int Tp = (T + L - 1) / L;
     c->Cpad = (n_channels + TILE_C - 1) / TILE_C * TILE_C;
-    c->Tpad = (T + KC - 1) / KC * KC;
+    c->Tpad = (Tp + KC - 1) / KC * KC;
     c->H = c->Tpad - 1;
     c->inc_a = (uint32_t)(int64_t)llround(s->audio_hz / s->output_rate * 4294967296.0);
     std::vector<uint32_t> inc(n_channels);
     for (int k = 0; k < n_channels; k++) inc[k] = (uint32_t)(int64_t)llround(offset_hz[k] / s->input_rate * 4294967296.0);
-    std::vector<float2> G((size_t)c->Tpad * c->Cpad, make_float2(0.f, 0.f));
-    for (int k = 0; k < T; k++)
+    const size_t branch = (size_t)c->Tpad * c->Cpad;
+    std::vector<float2> G(branch * L, make_float2(0.f, 0.f));
+    for (int k = 0; k < Tp; k++)
         for (int ch = 0; ch < n_channels; ch++) {
             uint32_t ph = inc[ch] * (uint32_t)k;
-            double a = 2.0 * M_PI * (double)ph / 4294967296.0;
-            G[(size_t)k * c->Cpad + ch] = make_float2((float)(h[k] * std::cos(a)), (float)(h[k] * std::sin(a)));
+            double a = 2.0 * M_PI * (double)ph / 4294967296.0, co = std::cos(a), si = std::sin(a);
+            for (int p = 0; p < L && k * L + p < T; p++) {
+                double hk = h[k * L + p];
+                G[p * branch + (size_t)k * c->Cpad + ch] = make_float2((float)(hk * co), (float)(hk * si));
+            }
         }
     if (c->allocs.upload(&c->d_G, G, c->stream) || c->allocs.upload(&c->d_inc, inc, c->stream)) return JAERO_E_CUDA;
     JB_CUDA(cudaStreamSynchronize(c->stream));
@@ -274,8 +311,8 @@ int jaero_chan_write_device(jaero_chan *c, const void *d_iq, size_t n)
     if (!c || (!d_iq && n)) { set_error("jaero_chan_write_device: null argument"); return JAERO_E_ARG; }
     if (n > ((size_t)1 << 31)) { set_error("jaero_chan_write_device: at most 2^31 samples per write"); return JAERO_E_ARG; }
     JB_CUDA(cudaSetDevice(c->device));
-    const long long N0 = c->n_in, D = c->D;
-    const long long m_first = (N0 + D - 1) / D, m_end = (N0 + (long long)n + D - 1) / D;
+    const long long N0 = c->n_in, L = c->L, Md = c->M;
+    const long long m_first = (L * N0 + Md - 1) / Md, m_end = (L * (N0 + (long long)n) + Md - 1) / Md;   // n_m inside the input
     const size_t M = (size_t)(m_end - m_first);
     c->n_out = M;
     if (n == 0) return JAERO_OK;
@@ -292,9 +329,9 @@ int jaero_chan_write_device(jaero_chan *c, const void *d_iq, size_t n)
     JB_CUDA(cudaGetLastError());
     c->launches++;
     if (M > 0) {
-        dim3 grid((unsigned)((M + TILE_M - 1) / TILE_M), (unsigned)(c->Cpad / TILE_C));
-        const long long off0 = m_first * D - N0 + c->H;
-        chan_ddc_kernel<<<grid, THREADS, 0, c->stream>>>(c->d_G, c->Cpad, c->Tpad, c->C, c->x[nb].ptr, off0, c->D, (int)M,
+        const size_t per_class = (M + L - 1) / L;                   // outputs of residue class 0, the largest
+        dim3 grid((unsigned)((per_class + TILE_M - 1) / TILE_M), (unsigned)(c->Cpad / TILE_C), (unsigned)std::min<size_t>(L, M));
+        chan_ddc_kernel<<<grid, THREADS, 0, c->stream>>>(c->d_G, c->Cpad, c->Tpad, c->C, c->x[nb].ptr, c->H - N0, c->M, c->L, (int)M,
                                                          (unsigned long long)m_first, c->d_inc, c->inc_a, c->gain, c->out.ptr, c->stride);
         JB_CUDA(cudaGetLastError());
         c->launches++;

@@ -273,15 +273,15 @@ def wideband_iq(envelopes, offsets_hz, input_rate, env_rate=48000.0, amplitudes=
     """Complex baseband IQ at input_rate carrying each circular envelope (oqpsk_envelope / msk_envelope, unit power, at
     env_rate) at its offset, plus complex AWGN, quantised as an SDR delivers it: [n, 2] int16 (cs16) or uint8 (cu8, the
     rtl_sdr format, x = ((u - 127.5) + j(v - 127.5)) * 256). Amplitudes (RMS, in cs16 LSB) default to 1000.
-    Each envelope is interpolated by zero-padding its FFT, so the result still loops seamlessly when every offset is a
+    Any input_rate >= env_rate works for which n = len(envelope) * input_rate / env_rate is an integer (2.048 MHz from
+    48 kHz, for example). Each envelope is interpolated by zero-padding its FFT to n, so the result still loops seamlessly when every offset is a
     multiple of env_rate / len(envelope). Noise: per-component variance N0 * input_rate / 2 with
     N0 = P / fb / 10^(ebn0_db / 10) of carrier `noise_ref` (P = its amplitude squared, fb its bit rate)."""
-    up = float(input_rate) / float(env_rate)
-    U = int(round(up))
-    assert abs(up - U) < 1e-9 and U >= 1, "input_rate must be an integer multiple of env_rate"
     L = len(envelopes[0])
     assert all(len(e) == L for e in envelopes)
-    n = L * U
+    nf = L * float(input_rate) / float(env_rate)
+    n = int(round(nf))
+    assert abs(nf - n) < 1e-9 * nf and n >= L, "len(envelope) * input_rate / env_rate must be an integer >= len(envelope)"
     amps = np.full(len(envelopes), 1000.0) if amplitudes is None else np.asarray(amplitudes, dtype=np.float64)
     fbs = np.broadcast_to(np.asarray(fb, dtype=np.float64), (len(envelopes),))
     t = np.arange(n, dtype=np.float64)
@@ -294,7 +294,7 @@ def wideband_iq(envelopes, offsets_hz, input_rate, env_rate=48000.0, amplitudes=
         Z[n - (L - h):] = E[h:]
         if L % 2 == 0:                                            # split the Nyquist bin so the result stays band-limited
             Z[h] = 0.5 * E[h]; Z[n - h] = 0.5 * E[h]
-        y = np.fft.ifft(Z) * U
+        y = np.fft.ifft(Z) * (n / L)                              # n / L = input_rate / env_rate, exact for an integer ratio
         x += a * y * np.exp(2j * np.pi * float(off) * t / float(input_rate))
     if ebn0_db is not None:
         rng = np.random.default_rng(seed)

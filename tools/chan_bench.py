@@ -1,15 +1,16 @@
 """Device channelizer measurement. One JSON line per configuration on stdout (and appended to --out if given).
 
-A  channelizer alone: 2.4 MHz cs16 IQ resident on the device (seeded noise), C = 192 and 4096 channels. 1 s of IQ warm-up,
-   then three timed repeats of 10 s of IQ each (1 s per write), CUDA events on the handle's stream. Reports ms per second
-   of IQ, the real-time factor, FP32 FLOP/s achieved from 8*T*C*M, output bytes, and a per-kernel breakdown taken with
-   torch.profiler in a separate pass.
-B  end to end, 4096 channels of OQPSK 10.5k: 2.4 MHz IQ carrying 64 distinct carriers, 64 channels tuned to each. Per 1 s
+A  channelizer alone: cs16 IQ at --input-rate (default 2.4 MHz) resident on the device (seeded noise), C = 192 and 4096
+   channels. 1 s of IQ warm-up, then three timed repeats of 10 s of IQ each (1 s per write), CUDA events on the handle's
+   stream. Reports ms per second of IQ, the real-time factor, FP32 FLOP/s achieved from 8*Tp*C*M_out (Tp taps per polyphase
+   branch, M_out outputs; Tp = T at integer rates), output bytes, and a per-kernel breakdown taken with torch.profiler in a
+   separate pass. Rates that are not a multiple of 48 kHz (2.048 MHz: L/M = 3/128) run the polyphase path.
+B  end to end, 4096 channels of OQPSK 10.5k: IQ at --input-rate carrying 64 distinct carriers, 64 channels tuned to each. Per 1 s
    step, on one stream: channelizer -> DemodBatch.write_device -> PChannelBatch.process_batch. Alternates, in the same
    process, with the same step fed device-resident PCM (a captured second of the channelizer's output), and with both
    inputs coming from pinned host memory (IQ through Channelizer.write, PCM through DemodBatch.write).
 
-python tools/chan_bench.py [--configs A,B] [--out FILE]   (needs a CUDA device; there is no CPU path)
+python tools/chan_bench.py [--configs A,B] [--input-rate HZ] [--out FILE]   (needs a CUDA device; there is no CPU path)
 """
 import argparse
 import json
@@ -28,8 +29,8 @@ import torch  # noqa: E402
 import jaero_b200 as jb  # noqa: E402
 from jaero_b200 import synth  # noqa: E402
 
-FS, FO, AUDIO = 2.4e6, 48000.0, 12000.0
-D = int(FS // FO)
+FO, AUDIO = 48000.0, 12000.0
+FS = 2.4e6                                                  # --input-rate
 
 
 def device_info():
@@ -60,6 +61,8 @@ def config_a(C, info, out, secs=10, repeats=3):
     ch = jb.Channelizer(off, FS, output_rate=FO, audio_hz=AUDIO, passband_hz=12000.0)
     ch.set_stream(s.cuda_stream)
     T = len(jb.channelizer_taps(FS, output_rate=FO, audio_hz=AUDIO, passband_hz=12000.0))
+    L, Mr = jb.channelizer_ratio(FS, output_rate=FO, audio_hz=AUDIO, passband_hz=12000.0)
+    Tp = (T + L - 1) // L
     torch.cuda.synchronize()
     ch.write_device(iq.data_ptr(), n1)                      # warm-up: 1 s of IQ
     ch.sync()
@@ -72,9 +75,9 @@ def config_a(C, info, out, secs=10, repeats=3):
         e1.record(s)
         e1.synchronize()
         times.append(e0.elapsed_time(e1) / secs)
-    M = n1 // D
+    M = n1 * L // Mr                                        # outputs per second of IQ
     st = stats(times)
-    flop = 8.0 * T * C * M
+    flop = 8.0 * Tp * C * M
     # per-kernel breakdown, profiler pass of its own (2 s of IQ)
     from torch.profiler import ProfilerActivity, profile
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
@@ -86,7 +89,7 @@ def config_a(C, info, out, secs=10, repeats=3):
         if "chan_" in e.key:
             name = "chan_ddc_kernel" if "ddc" in e.key else "chan_convert_kernel"
             kern[name] = round(e.device_time_total / 1000.0 / 2, 3)   # ms per second of IQ
-    rec = dict(config="A", channels=C, input_rate=FS, output_rate=FO, taps=T, iq_format="cs16", secs_per_repeat=secs,
+    rec = dict(config="A", channels=C, input_rate=FS, output_rate=FO, taps=T, ratio=[L, Mr], taps_per_phase=Tp, iq_format="cs16", secs_per_repeat=secs,
                ms_per_s_iq=st, realtime_factor=1000.0 / st["median"], fp32_tflops=flop / (st["median"] * 1e-3) / 1e12,
                flop_per_s_iq=flop, output_bytes_per_s_iq=C * M * 2, input_bytes_per_s_iq=n1 * 4,
                kernel_ms_per_s_iq=kern, launches_per_write=2, **info)
@@ -182,7 +185,10 @@ def main():
     ap.add_argument("--configs", default="A,B")
     ap.add_argument("--out", default=None)
     ap.add_argument("--secs", type=int, default=10)
+    ap.add_argument("--input-rate", type=float, default=2.4e6)
     a = ap.parse_args()
+    global FS
+    FS = a.input_rate
     if not torch.cuda.is_available() or jb.lib().jaero_device_count() < 1:
         sys.exit("chan_bench: needs a CUDA device (there is no CPU path)")
     info = device_info()
